@@ -12,6 +12,7 @@ arithmetic of the reference's own GPU path (cuDNN TF32 convs); ``--math bf16`` /
 One "step" = one complete ``sample()`` call (initial noise, 100 reverse iterations, final all-gather when N > 1).
 
   python bench.py --gpus 1 --steps 5 --warmup 3              # this framework (CUDA engine through the C ABI)
+  python bench.py --gpus 1 --steps 5 --warmup 3 --dump-outputs OUT   # + the last timed step's samples as OUT/x0.npy
   python bench.py --impl reference --steps 2 --warmup 1      # CPU arm: the reference's algorithm (oracle port) on host cores
   torchrun ... bench.py --gpus N ...                         # one rank per GPU, NCCL
 
@@ -270,6 +271,23 @@ def gpu_eager_baseline(agent, prior_dev, kw, B):
             os.environ["CDS_BACKEND"] = old
 
 
+def dump_outputs(out_dir, arrays, budget=64_000_000, seed=0):
+    """Each array -> out_dir/<name>.npy in float32.  An array larger than its share of the byte budget keeps a fixed sample
+    of its rows (trajectories): the same seeded choice, in ascending order, on every run with the same arguments."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    share = budget // len(arrays) - 4096                              # room for the .npy header
+    for name, a in arrays.items():
+        a = a.float()
+        n, rows = a.shape[0], max(1, share // (a[0].numel() * 4))
+        if n > rows:
+            keep = torch.randperm(n, generator=torch.Generator().manual_seed(seed))[:rows].sort().values
+            a = a[keep]
+            log(f"dump: {name} sampled to {rows} of {n} rows (seed {seed})")
+        np.save(os.path.join(out_dir, name + ".npy"), a.numpy())
+        log(f"dump: {os.path.join(out_dir, name + '.npy')} {tuple(a.shape)} float32")
+
+
 # ------------------------------------------------------------------------------------------ main
 def main():
     ap = argparse.ArgumentParser()
@@ -285,7 +303,14 @@ def main():
     ap.add_argument("--no-other-configs", action="store_true")
     ap.add_argument("--no-eager-baseline", action="store_true")
     ap.add_argument("--cpu-sample-batch", type=int, default=256, help="trajectories per step of the CPU arm (bounded sample)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (float32; trajectories beyond a 64 MB budget "
+                         "are replaced by a fixed seeded sample of them), so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the CUDA path's samples; it does not apply to --impl reference")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -304,13 +329,13 @@ def main():
         sb = args.cpu_sample_batch
         while sb > 32 and (args.steps + args.warmup) * (sb / 100.0) > 240:      # ~100 traj/s on 16 threads -> seconds per step
             sb //= 2
-        value, sec, sb = cpu_reference_arm(max(args.steps, 1), max(args.warmup, 0), sample_batch=sb)
+        value, sec, sb = cpu_reference_arm(args.steps, max(args.warmup, 0), sample_batch=sb)
         cores = torch.get_num_threads()
         config = dict(config, cpu_sample_batch=sb,
                       note=f"CPU arm: every step runs the full 100-step sample() on {sb} of the {args.batch} trajectories "
                            "(bounded sample; throughput in trajectories/s is batch-size independent to first order)")
         line = {"impl": "reference", "metric": "sampled trajectories/sec (H=32, 100 DDPM steps)", "value": value,
-                "unit": "trajectories/s", "n_gpus": args.gpus, "steps": max(args.steps, 1), "warmup": max(args.warmup, 0),
+                "unit": "trajectories/s", "n_gpus": args.gpus, "steps": args.steps, "warmup": max(args.warmup, 0),
                 "ms_per_step": sec * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
                 "dtype": "f32", "data": "synthetic", "config": config,
                 "cpu_baseline": {"value": value, "unit": "trajectories/s", "cores": cores, "kind": "port",
@@ -347,11 +372,14 @@ def main():
     gathered = torch.empty(world * B, H, D, device=device) if world > 1 else None
     kw = dict(solver="ddpm", n_samples=B, sample_steps=S_STEPS, temperature=0.5)
     torch.manual_seed(2 + rank)
+    last = {}
 
     def step_resident():
         x0, _ = agent.sample(prior_dev, **kw)
         if world > 1:
             dist.all_gather_into_tensor(gathered, x0)      # the one collective of the path: finished samples
+        if args.dump_outputs:
+            last["x0"] = x0                                # a fresh tensor per call: later calls do not overwrite it
         return x0
 
     def step_e2e():
@@ -379,6 +407,8 @@ def main():
             row0 = len(clk.rows)
             runtime.STATS["loop_events"] = []
             ms = timed(step_resident, args.steps)
+            if args.dump_outputs and rank == 0:       # copied now: the e2e steps below reuse the gather buffer
+                outputs = {"x0": (gathered if world > 1 else last["x0"]).cpu()}
             row1 = len(clk.rows)
             extended = 0
             t_ext = time.time()
@@ -496,6 +526,9 @@ def main():
         cpu_baseline = {"value": v, "unit": "trajectories/s", "cores": torch.get_num_threads(), "kind": "port",
                         "sample": f"one full 100-step sample() on {sb} trajectories ({sec:.1f} s), oracle port of the "
                                   f"reference algorithm on torch CPU fp32"}
+
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, outputs)
 
     if saved_stdout is not None:
         sys.stdout.flush()

@@ -66,6 +66,14 @@ NETS = {
 NET_BATCH = 3
 
 
+def module_names(m):
+    """(public instance attribute names, names the class defines below nn.Module) of a module, both sorted: what an instance
+    offers the lowering besides its sub-modules, parameters and buffers."""
+    mro = type(m).__mro__
+    own = {k for base in mro[:mro.index(torch.nn.Module)] for k in vars(base) if not (k.startswith("__") and k.endswith("__"))}
+    return sorted(k for k in vars(m) if not k.startswith("_")), sorted(own)
+
+
 def net_inputs(case: dict, seed: int = 1):
     g = torch.Generator().manual_seed(seed)
     x = torch.randn((NET_BATCH, *case["x"]), generator=g)

@@ -266,9 +266,54 @@ def gen_edm():
     print("edm.npz", len(out))
 
 
+def module_tree(net):
+    """[path, class module, class name, {param: shape}, {buffer: shape}, {plain attribute: value}, public attribute names,
+    class-defined names] per sub-module, in ``named_modules`` order: everything structural the lowering can read from an
+    instance.  The two name lists are recorded for the reference's own classes only (None for torch classes)."""
+    plain = (int, float, bool, str, type(None))
+    rows = []
+    for path, m in net.named_modules():
+        attrs = {k: list(v) if isinstance(v, tuple) else v for k, v in vars(m).items()
+                 if not k.startswith("_") and k != "training"
+                 and (isinstance(v, plain) or isinstance(v, (tuple, list)) and all(isinstance(e, plain) for e in v))}
+        names = cases.module_names(m) if type(m).__module__.startswith("cleandiffuser.") else (None, None)
+        rows.append([path, type(m).__module__, type(m).__name__,
+                     {k: list(p.shape) for k, p in m.named_parameters(recurse=False)},
+                     {k: list(b.shape) for k, b in m.named_buffers(recurse=False)}, attrs, *names])
+    return rows
+
+
+def diffusion_layout():
+    """{module: {class name: defining module}} for ``cleandiffuser.diffusion`` and each of its sub-modules: every
+    reference class bound there, defined or imported."""
+    import importlib
+    import pkgutil
+    import cleandiffuser.diffusion as pkg
+    layout = {}
+    for name in [pkg.__name__] + [f"{pkg.__name__}.{m.name}" for m in pkgutil.iter_modules(pkg.__path__)]:
+        mod = importlib.import_module(name)
+        layout[name] = {k: v.__module__ for k, v in vars(mod).items()
+                        if isinstance(v, type) and v.__module__.startswith("cleandiffuser.")}
+    return layout
+
+
+def gen_reference_modules():
+    """The module trees of the reference's own backbone instances (the NETS cases and the sampler nets) and the layout of
+    its ``diffusion`` package, so that tests/test_reference_instances_cpu.py can rebuild instances with the reference's
+    structure and class identity, and a package with the reference's layout for ``install()``."""
+    import json
+    out = {}
+    for name, case in list(cases.NETS.items()) + [("sampler/" + k, v) for k, v in cases.SAMPLER_NETS.items()]:
+        out[name] = np.array(json.dumps(module_tree(getattr(ref_nn, case["cls"])(**case["ctor"])), separators=(",", ":")))
+    out["layout/diffusion"] = np.array(json.dumps(diffusion_layout(), separators=(",", ":")))
+    np.savez_compressed(os.path.join(HERE, "reference_modules.npz"), **out)
+    print("reference_modules.npz", len(out))
+
+
 if __name__ == "__main__":
     torch.set_num_threads(1)
     only = sys.argv[1:]
-    for fn in (gen_tables, gen_nets, gen_samplers, gen_consistency, gen_edm, gen_guided, gen_legacy, gen_rf, gen_legacy_edm):
+    for fn in (gen_tables, gen_nets, gen_samplers, gen_consistency, gen_edm, gen_guided, gen_legacy, gen_rf, gen_legacy_edm,
+               gen_reference_modules):
         if not only or fn.__name__[4:] in only:
             fn()
