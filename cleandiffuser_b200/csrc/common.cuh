@@ -28,6 +28,16 @@ __device__ __forceinline__ VecRef resolve(const cds_vec& v, int iter) {
   return r;
 }
 
+// mean of v[first .. first + n).  The tensor-core kernels subtract it from the bias of a GroupNorm group when they stage the
+// per-column constants: GroupNorm does not change under a common shift of its group, and with the group's common offset gone
+// the single-pass moments E[y^2] - E[y]^2 in fp32 no longer cancel (a bias of 256 group sigmas cost ~1e-2 in rstd).  Every
+// column of a group sums the same values in the same order, so the shift is bit-identical across the group.
+__device__ __forceinline__ float group_mean(const float* v, int first, int n) {
+  float s = 0.f;
+  for (int j = 0; j < n; ++j) s += __ldg(v + first + j);
+  return s / (float)n;
+}
+
 // activations; formulas follow ATen's fp32 CUDA/CPU definitions
 __device__ __forceinline__ float act_mish(float x) {
   // x * tanh(softplus(x)), softplus with torch's threshold of 20

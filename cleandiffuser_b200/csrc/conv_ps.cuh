@@ -229,7 +229,7 @@ conv_ps_kernel(const __grid_constant__ ConvPsParams p, const int* __restrict__ i
       const float* hstep = p.shift.step ? p.shift.step + (int64_t)iter * p.shift.step_stride : nullptr;
       for (int n = threadIdx.x; n < N; n += kPsEpiThreads) {
         const int c = n_off + n;
-        s_col[0][n] = bstep ? __ldg(bstep + c) : 0.f;
+        s_col[0][n] = bstep ? __ldg(bstep + c) - group_mean(bstep, c - c % NH, NH) : 0.f;   // (a group = NH = C_out / 8 columns)
         s_col[1][n] = __ldg(p.gn_gamma + c);
         s_col[2][n] = __ldg(p.gn_beta + c);
         s_col[3][n] = hstep ? __ldg(hstep + c) : 0.f;

@@ -162,6 +162,15 @@ __global__ void __launch_bounds__(kThreads) conv_gemm_f32_kernel(const cds_conv_
 
   // ---- accumulators (+bias) -> shared tile -------------------------------------------------------
   const VecRef bias = resolve(p.bias, iter);
+  // GroupNorm layers: the step bias minus its group mean (group_mean, common.cuh) -- the normalised output is the same, and the
+  // fp32 mean of the statistics pass no longer carries the rounding of a large common offset
+  float bias_shift[TN];
+#pragma unroll
+  for (int j = 0; j < TN; ++j) {
+    const int ng = n0 + tx * TN + j;
+    const int gcpg = p.groups > 0 ? p.C_out / p.groups : 0;
+    bias_shift[j] = (gcpg && bias.step && ng < N_total) ? group_mean(bias.step, ng - ng % gcpg, gcpg) : 0.f;
+  }
 #pragma unroll
   for (int i = 0; i < 8; ++i) {
     int m = ty * 8 + i;
@@ -172,7 +181,11 @@ __global__ void __launch_bounds__(kThreads) conv_gemm_f32_kernel(const cds_conv_
       int n = tx * TN + j;
       int ng = n0 + n;
       float v = acc[i][j];
-      if (r < rows && ng < N_total && bias.present()) v += bias.at(b, ng % p.C_out);
+      if (r < rows && ng < N_total && bias.present()) {
+        const int c = ng % p.C_out;
+        if (bias.step) v += __ldg(bias.step + c) - bias_shift[j];
+        if (bias.sample) v += __ldg(bias.sample + (int64_t)b * bias.sample_stride + c);
+      }
       Cs[m * (BN + 1) + n] = v;
     }
   }

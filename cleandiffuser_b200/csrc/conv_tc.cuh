@@ -434,10 +434,11 @@ conv_tc_kernel(const __grid_constant__ ConvTcParams p, const int* __restrict__ i
       const float* sstep = p.scale.step ? p.scale.step + (int64_t)iter * p.scale.step_stride : nullptr;
       const float* hstep = p.shift.step ? p.shift.step + (int64_t)iter * p.shift.step_stride : nullptr;
       const bool scale_any = p.scale.step || p.scale.sample;
+      const int cpg = p.groups > 0 ? p.C_out / p.groups : 0;
       for (int n = threadIdx.x; n < Cfg::kCols; n += kTcEpiThreads) {
         const bool real = first + n < n_real;
         const int c = real ? (first + n) % p.C_out : 0;
-        s_col[0][n] = (real && bstep) ? __ldg(bstep + c) : 0.f;
+        s_col[0][n] = (real && bstep) ? __ldg(bstep + c) - (cpg ? group_mean(bstep, c - c % cpg, cpg) : 0.f) : 0.f;
         s_col[1][n] = (real && p.groups > 0) ? __ldg(p.gn_gamma + c) : 1.f;
         s_col[2][n] = (real && p.groups > 0) ? __ldg(p.gn_beta + c) : 0.f;
         s_col[3][n] = sstep ? (real ? __ldg(sstep + c) : 0.f) : (scale_any ? 0.f : 1.f);
